@@ -1,8 +1,13 @@
 #!/usr/bin/env python3
 """bench.py — tuples/s of the tree-walk hot path on BASELINE.json's headline configuration.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR (ours): after the timed steps, rank 0 writes what its last step returned for a fixed, seeded
+  sample of DUMP_TUPLES tuples (all of them when fewer are requested): DIR/scores.npy (float32), DIR/labels.npy
+  (0/1 as float32) and DIR/tuple_index.npy (float64, the sampled tuple indices).  The inputs depend only on the
+  arguments, so two builds run with the same arguments can be compared file for file.
 
 ours: one "step" = one pass of the walk kernel (through the C ABI, libdte.so) over one batch of
   synthetic tuples already resident in HBM.  N=1 workload = BASELINE configs[2]
@@ -36,6 +41,8 @@ N_FULL = 50_000_000
 MISSING_PPM = 10000
 SEED_TUPLES = 0x7091E5
 SM_COUNT = 148
+DUMP_TUPLES = 1 << 20           # --dump-outputs sample: 16 MiB of .npy files
+DUMP_SEED = 0xD0
 
 
 def algorithmic_bytes_per_tuple(T, D, F):
@@ -240,6 +247,23 @@ def sample_indices(n, k):
     return np.unique(np.concatenate([np.arange(min(64, n)), np.arange(0, n, max(1, n // max(1, k - 64)))]))[:k]
 
 
+def dump_outputs(out_dir, d_scores, d_labels, n, n_requested):
+    """Scores and labels of the last timed step for a fixed, seeded sample of its n tuples (see --dump-outputs).  The
+    sample is drawn from the requested tuple count, so a step shortened for lack of device memory keeps the sampled
+    tuples that it still holds."""
+    import torch
+    if n_requested <= DUMP_TUPLES:
+        idx = np.arange(n)
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n_requested, DUMP_TUPLES, replace=False))
+        idx = idx[idx < n]
+    sel = torch.from_numpy(idx).to(d_scores.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scores.npy"), d_scores[sel].cpu().numpy())
+    np.save(os.path.join(out_dir, "labels.npy"), d_labels[sel].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "tuple_index.npy"), idx.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -255,10 +279,15 @@ def main():
     ap.add_argument("--trees", type=int, default=T_TREES)
     ap.add_argument("--depth", type=int, default=DEPTH)
     ap.add_argument("--features", type=int, default=FEATS)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's scores and labels as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs dumps the GPU path; the reference arm times a CPU sample sized by the clock")
         return run_reference(args)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -351,6 +380,8 @@ def main():
         evs[i + 1].record()
     barrier()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:                    # before any later leg reuses d_s / d_l
+        dump_outputs(args.dump_outputs, d_s, d_l, n, args.tuples or N_FULL)
     total_ms = evs[0].elapsed_time(evs[-1])
     per_launch_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
     launches = e.info()["kernel_launches"] - launches0
